@@ -4,6 +4,7 @@
 
     python bench.py --gpus 1 --steps 5 --warmup 3                # B200 engine (default)
     python bench.py --impl reference --gpus 1 --steps 5 --warmup 3   # the reference's CPU path
+    python bench.py --gpus 1 --steps 5 --warmup 3 --dump-outputs DIR   # also write the last step's results
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...   # document-sharded
 
 A "step" is one batch of 64 queries x 32 tokens through the whole hot path.  `value` is
@@ -14,6 +15,11 @@ copies inside the timed region.  One JSON line on stdout.
 
 Parity is part of the line: `parity_sample` runs the CPU oracle on the first queries of a batch, at
 any number of GPUs, and classifies every difference between the engine's id lists and the oracle's.
+
+`--dump-outputs DIR` writes what the timed path returned in its last step -- DIR/ids.npy (float64 [B, top_k],
+-1 past the count), DIR/scores.npy (float32 [B, top_k], -inf past the count), DIR/counts.npy (float64 [B]) --
+so that two builds run with the same arguments (hence the same seeded index and queries) can be compared output for
+output.
 """
 
 from __future__ import annotations
@@ -34,6 +40,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 CONFIGS = {
@@ -319,6 +326,7 @@ def run_b200(args) -> dict:
     gathered = torch.empty((world, B, lay.R, 16), dtype=torch.uint8, device=device)
     keys = torch.empty((B, lay.R), dtype=torch.int64, device=device)
     all_keys = torch.empty((world, B, lay.R), dtype=torch.int64, device=device)
+    last = [ids, scores, counts]  # what the timed path returned in its latest step
     stage_names = ["centroid_scores", "probe", "candidates", "approx", "select", "maxsim", "final"]
     if world > 1:
         stage_names = ["centroid_scores", "probe", "candidates", "approx", "select", "exchange_keys", "maxsim", "final"]
@@ -377,7 +385,7 @@ def run_b200(args) -> dict:
                 e0 = torch.cuda.Event(enable_timing=True)
                 e0.record()
                 events.append(e0)
-            didx.search_sharded(comm, n_groups, qb, params)
+            last[:] = didx.search_sharded(comm, n_groups, qb, params)
             if events is not None:
                 e1 = torch.cuda.Event(enable_timing=True)
                 e1.record()
@@ -400,6 +408,8 @@ def run_b200(args) -> dict:
         all_events.append(ev)
     barrier()
     t_wall = time.time() - t_wall0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)
     total_ms = all_events[0][0].elapsed_time(all_events[-1][-1])
     stage_ms = [0.0] * len(stage_names)
     for ev in all_events:
@@ -611,6 +621,13 @@ def run_b200(args) -> dict:
         dist.barrier()
         dist.destroy_process_group()
     return out if rank == 0 else {}
+
+
+def dump_outputs(out_dir: str, ids: torch.Tensor, scores: torch.Tensor, counts: torch.Tensor) -> None:
+    """The results of one step as .npy files: ids and counts as float64 (exact for any doc id below 2**53)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t, dt in (("ids", ids, np.float64), ("scores", scores, np.float32), ("counts", counts, np.float64)):
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.cpu().numpy().astype(dt))
 
 
 def count_launches(world: int, approx: str) -> int:
@@ -985,7 +1002,7 @@ def run_reference(args) -> dict:
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps (at least 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", choices=["b200", "reference"], default="b200")
     ap.add_argument("--config", choices=list(CONFIGS), default="cfg3")
@@ -998,7 +1015,13 @@ def main() -> None:
                          "shards that fit the per-GPU budget)")
     ap.add_argument("--approx", choices=["two-pass", "direct"], default="two-pass",
                     help="approximate stage: exact two-pass pruning (default) or the one-pass A/B alternative")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the ids, scores and counts the timed path returned in its last step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the engine's results: it needs --impl b200")
     # keep stdout clean for the ONE JSON line: NCCL / libraries may print to fd 1
     sys.stdout.flush()
     real_stdout = os.dup(1)

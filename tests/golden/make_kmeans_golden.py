@@ -1,13 +1,13 @@
-"""Mint tests/golden/kmeans_ref.pt by running the REFERENCE's own k-means code.
+"""Mint tests/golden/kmeans_ref.pt and kmeans_ref_fresh.pt by running the REFERENCE's own k-means code.
 
 The Lloyd loop the reference layers on the (absent) third-party `fastkmeans` package lives in
-/root/reference/python/fast_plaid/search/kmeans.py:60-223 and is plain PyTorch.  This script
+python/fast_plaid/search/kmeans.py:60-223 of the reference and is plain PyTorch.  This script
 imports that file unmodified -- only `fastkmeans` itself is stubbed with an empty base class --
 seeds the RNG exactly as `FastKMeans.train` does (kmeans.py:236-238) and records inputs and
 outputs.  tests/test_oracle.py then requires oracle/index_oracle.py::kmeans to reproduce the
 recorded centroids, which pins that part of the oracle on reference outputs.
 
-Run in the build container (needs /root/reference):  python tests/golden/make_kmeans_golden.py
+    python tests/golden/make_kmeans_golden.py <checkout of the reference fast-plaid sources>
 """
 
 import importlib.util
@@ -18,11 +18,12 @@ import types
 import numpy as np
 import torch
 
-REF = "/root/reference/python/fast_plaid/search/kmeans.py"
-OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "kmeans_ref.pt")
+HERE = os.path.dirname(os.path.abspath(__file__))
+OUT = os.path.join(HERE, "kmeans_ref.pt")
+OUT_FRESH = os.path.join(HERE, "kmeans_ref_fresh.pt")
 
 
-def load_reference_kmeans():
+def load_reference_kmeans(ref_root: str):
     stub = types.ModuleType("fastkmeans")
 
     class FastKMeans:  # the third-party base class; never instantiated here
@@ -30,7 +31,8 @@ def load_reference_kmeans():
 
     stub.FastKMeans = FastKMeans
     sys.modules.setdefault("fastkmeans", stub)
-    spec = importlib.util.spec_from_file_location("ref_kmeans", REF)
+    path = os.path.join(ref_root, "python", "fast_plaid", "search", "kmeans.py")
+    spec = importlib.util.spec_from_file_location("ref_kmeans", path)
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
     return mod
@@ -47,9 +49,9 @@ def run_case(mod, data_f16: torch.Tensor, k: int, niters: int, seed: int, mppc: 
     return centroids, labels
 
 
-def main():
+def main(ref_root: str):
     torch.set_num_threads(1)  # the fixture must not depend on the blocking of a threaded GEMM
-    mod = load_reference_kmeans()
+    mod = load_reference_kmeans(ref_root)
     g = torch.Generator().manual_seed(2024)
     cases = []
     # (n, dim, k, niters, seed, max_points_per_centroid)
@@ -67,7 +69,19 @@ def main():
                           "torch " + torch.__version__ + ", CPU, 1 thread",
                 "cases": cases}, OUT)
     print("wrote", OUT, os.path.getsize(OUT), "bytes")
+    # a problem drawn apart from the mixtures above: plain normalised noise
+    g = torch.Generator().manual_seed(99)
+    x = torch.nn.functional.normalize(torch.randn(1500, 24, generator=g), dim=-1).half()
+    k, niters, seed, mppc = 32, 3, 5, 256
+    c, _ = run_case(mod, x, k, niters, seed, mppc)
+    torch.save({"source": "reference python/fast_plaid/search/kmeans.py::_kmeans_torch_double_chunked, "
+                          "torch " + torch.__version__ + ", CPU, 1 thread",
+                "case": dict(data=x, k=k, niters=niters, seed=seed, max_points_per_centroid=mppc, centroids=c)},
+               OUT_FRESH)
+    print("wrote", OUT_FRESH, os.path.getsize(OUT_FRESH), "bytes")
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2:
+        raise SystemExit(__doc__)
+    main(sys.argv[1])

@@ -9,6 +9,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 import torch
 
@@ -33,6 +34,28 @@ def test_product_arm_has_no_cpu_fallback():
                        capture_output=True, text=True, timeout=300)
     assert r.returncode != 0
     assert "CUDA" in (r.stderr + r.stdout)
+
+
+def test_steps_below_one_are_refused():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"],
+                       capture_output=True, text=True, timeout=300)
+    assert r.returncode == 2 and "--steps" in r.stderr
+
+
+def test_dump_outputs_writes_float_arrays_of_the_results(tmp_path):
+    sys.path.insert(0, ROOT)
+    import bench
+
+    ids = torch.tensor([[7, 2**40 + 3, -1], [0, -1, -1]])
+    scores = torch.tensor([[31.5, 30.25, float("-inf")], [12.0, float("-inf"), float("-inf")]])
+    counts = torch.tensor([2, 1], dtype=torch.int32)
+    out = tmp_path / "dump"
+    bench.dump_outputs(str(out), ids, scores, counts)
+    got = {p.stem: np.load(p) for p in out.iterdir()}
+    assert set(got) == {"ids", "scores", "counts"}
+    assert got["ids"].dtype == np.float64 and got["ids"].tolist() == ids.tolist()
+    assert got["scores"].dtype == np.float32 and got["scores"].tolist() == scores.tolist()
+    assert got["counts"].dtype == np.float64 and got["counts"].tolist() == counts.tolist()
 
 
 def test_bench_configs_cover_the_baseline_configs():

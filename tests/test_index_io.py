@@ -1,12 +1,11 @@
-"""Index directory layout: the product's builder/reader against the oracle's builder and --
-when /root/reference is mounted -- against the reference's own Python loader."""
+"""Index directory layout: the product's builder/reader against the oracle's builder and against what the
+reference's own Python loader read from a directory our builder wrote."""
 
 from __future__ import annotations
 
 import json
 import os
-import sys
-import types
+from io import BytesIO
 
 import numpy as np
 import pytest
@@ -75,32 +74,31 @@ def test_ivf_lists_are_sorted_unique_and_consistent(built):
         assert set(lst.tolist()) == set(tok2doc[data.doc_codes == c].tolist())
 
 
-REF_PY = "/root/reference/python"
+LOADER_GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "reference_loader.pt")
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_PY), reason="reference tree not mounted (GPU box)")
-def test_reference_loader_reads_our_directory_identically(built, monkeypatch):
+def _write_files(path: str, files: dict[str, bytes]) -> None:
+    for name, data in files.items():
+        with open(os.path.join(path, name), "wb") as f:
+            f.write(data)
+
+
+def test_reference_loader_reads_our_directory_identically(built, tmp_path):
     """Pin the on-disk format against the reference's OWN loader
-    (python/fast_plaid/search/load.py:220-322).  Its module imports the Rust extension and the
-    third-party fastkmeans at import time; both are stubbed -- the loader code that runs is the
-    reference's, unmodified, read from /root/reference."""
-    path, _ = built
-    stub = types.ModuleType("fast_plaid.fast_plaid_rust")
-    pkg = types.ModuleType("fast_plaid")
-    pkg.__path__ = [os.path.join(REF_PY, "fast_plaid")]
-    pkg.fast_plaid_rust = stub
-    srch = types.ModuleType("fast_plaid.search")
-    srch.__path__ = [os.path.join(REF_PY, "fast_plaid", "search")]
-    monkeypatch.setitem(sys.modules, "fast_plaid", pkg)
-    monkeypatch.setitem(sys.modules, "fast_plaid.fast_plaid_rust", stub)
-    monkeypatch.setitem(sys.modules, "fast_plaid.search", srch)
-    import importlib.util
-
-    spec = importlib.util.spec_from_file_location("fast_plaid.search.load",
-                                                  os.path.join(REF_PY, "fast_plaid", "search", "load.py"))
-    ref_load = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref_load)
-    ref = ref_load._load_index_tensors_cpu(index_path=path)
+    (python/fast_plaid/search/load.py:220-322).  tests/golden/reference_loader.pt holds a directory written by our
+    builder, the tensors the reference's loader read from it and the merged mmap cache it wrote there
+    (tests/golden/make_loader_golden.py); our reader must return the same tensors."""
+    blob = torch.load(LOADER_GOLDEN, weights_only=False)
+    # the builder still writes that directory: same files, same array dtypes (embeddings.npy is not stored)
+    built_path, _ = built
+    assert set(os.listdir(built_path)) - {"embeddings.npy"} == set(blob["files"])
+    for name in blob["files"]:
+        if name.endswith(".npy"):
+            stored = np.load(BytesIO(blob["files"][name]))
+            assert np.load(os.path.join(built_path, name)).dtype == stored.dtype, name
+    path = str(tmp_path)
+    _write_files(path, blob["files"])
+    ref = blob["reference"]
     ours = store.read_index(path)
     n_tok = int(ours.doc_lengths.sum())
     assert ref["nbits"] == ours.nbits
@@ -114,10 +112,10 @@ def test_reference_loader_reads_our_directory_identically(built, monkeypatch):
     assert torch.equal(ref["doc_residuals"][:n_tok], ours.doc_residuals)
     assert ref["doc_codes"].shape[0] - n_tok == int(ours.doc_lengths.max() - ours.doc_lengths[-1])
     # the merged mmap cache the reference wrote does not confuse our reader
+    assert {"merged_codes.npy", "merged_residuals.npy"} <= set(blob["loader_files"])
+    _write_files(path, blob["loader_files"])
     again = store.read_index(path)
     assert torch.equal(again.doc_codes, ours.doc_codes)
-    for f in ("merged_codes.npy", "merged_residuals.npy", "merged_codes.manifest.json", "merged_residuals.manifest.json"):
-        os.remove(os.path.join(path, f))
 
 
 def test_pack_buckets_is_the_reference_bit_order():

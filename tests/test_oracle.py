@@ -200,19 +200,14 @@ def test_kmeans_restatement_reproduces_reference_outputs():
         assert torch.equal(got, c["centroids"]), float((got - c["centroids"]).abs().max())
 
 
-@pytest.mark.skipif(not os.path.isfile("/root/reference/python/fast_plaid/search/kmeans.py"),
-                    reason="reference tree not mounted (GPU box)")
-def test_kmeans_restatement_against_the_live_reference_code():
-    """Same check against the reference file itself (fresh random problem, not the fixture)."""
-    import importlib.util
-    import sys
-
-    sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
-    import make_kmeans_golden as mk
+def test_kmeans_restatement_reproduces_reference_outputs_on_fresh_data():
+    """Same check on a problem drawn apart from the fixture above (plain normalised noise, k=32), recorded in
+    tests/golden/kmeans_ref_fresh.pt by tests/golden/make_kmeans_golden.py."""
     from oracle import index_oracle as io
 
-    mod = mk.load_reference_kmeans()
-    g = torch.Generator().manual_seed(99)
-    x = torch.nn.functional.normalize(torch.randn(1500, 24, generator=g), dim=-1).half()
-    ref_c, _ = mk.run_case(mod, x, 32, 3, 5, 256)
-    assert torch.equal(io.kmeans(x, 32, 3, 5, 256), ref_c)
+    blob = torch.load(os.path.join(os.path.dirname(__file__), "golden", "kmeans_ref_fresh.pt"), weights_only=False)
+    assert "reference" in blob["source"]
+    c = blob["case"]
+    assert c["data"].shape == (1500, 24) and c["k"] == 32
+    got = io.kmeans(c["data"], c["k"], c["niters"], c["seed"], c["max_points_per_centroid"])
+    assert torch.equal(got, c["centroids"]), float((got - c["centroids"]).abs().max())
