@@ -84,11 +84,13 @@ __device__ __forceinline__ uint32_t en_sw_off(int r, int c) {
 
 // KMEANS = false: code = argmax_k fp16(<x, c_k>)                      (index-build encode)
 // KMEANS = true : code = argmax_k (<x, c_k> + bias[k]) in fp32, bias[k] = -|c_k|^2 / 2, i.e. the nearest centroid
-//                 by squared distance (the assignment step of Lloyd's algorithm, kmeans.py:153-160)
+//                 by squared distance (the assignment step of Lloyd's algorithm, kmeans.py:153-160); `best`
+//                 (optional) receives that maximum, from which the caller gets min_k |x - c_k|^2 = |x|^2 - 2 best
 template <bool KMEANS>
 __global__ void __launch_bounds__(EN_THREADS, 1)
 encode_assign_kernel(const __grid_constant__ CUtensorMap tmap_c, int K, const __half* __restrict__ X, int64_t n,
-                     int32_t* __restrict__ codes, int n_ctiles, const float* __restrict__ bias) {
+                     int32_t* __restrict__ codes, int n_ctiles, const float* __restrict__ bias,
+                     float* __restrict__ best_out) {
   __shared__ float s_bias[4][2][128];  // per epilogue warp and accumulator: the tile's biases
   extern __shared__ unsigned char smem_dyn[];
   const uint32_t dyn_addr = smem_u32(smem_dyn);
@@ -218,7 +220,10 @@ encode_assign_kernel(const __grid_constant__ CUtensorMap tmap_c, int K, const __
         __syncwarp();
         if (lane == 0) en_mbar_arrive(bar_tempty + 8 * acc);
       }
-      if (tok < n) codes[tok] = best_k;
+      if (tok < n) {
+        codes[tok] = best_k;
+        if (KMEANS && best_out) best_out[tok] = best;
+      }
     }
     it += uint32_t(n_ctiles);
   }
@@ -270,9 +275,11 @@ typedef CUresult (*en_encode_tiled_fn)(CUtensorMap*, CUtensorMapDataType, cuuint
 
 }  // namespace
 
-// tensor map of the centroid table + launch of the assign kernel (shared by fpb_encode and fpb_kmeans_assign)
+// tensor map of the centroid table + launch of the assign kernel (shared by fpb_encode, fpb_kmeans_assign and
+// fpb_nearest_centroid; d_best needs d_bias)
 static int launch_assign(int device, int64_t n_centroids, const void* d_centroids, const void* d_tokens,
-                         int64_t n_tokens, int32_t* d_codes, const float* d_bias, cudaStream_t st, const char* who) {
+                         int64_t n_tokens, int32_t* d_codes, const float* d_bias, float* d_best, cudaStream_t st,
+                         const char* who) {
   void* fn = nullptr;
   cudaDriverEntryPointQueryResult qres;
   if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess || !fn ||
@@ -302,12 +309,12 @@ static int launch_assign(int device, int64_t n_centroids, const void* d_centroid
     FPB_CUDA_CHECK(cudaFuncSetAttribute(encode_assign_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, EnSmem::bytes));
     encode_assign_kernel<true><<<blocks, EN_THREADS, EnSmem::bytes, st>>>(tm, int(n_centroids),
                                                                          static_cast<const __half*>(d_tokens), n_tokens,
-                                                                         d_codes, n_ctiles, d_bias);
+                                                                         d_codes, n_ctiles, d_bias, d_best);
   } else {
     FPB_CUDA_CHECK(cudaFuncSetAttribute(encode_assign_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, EnSmem::bytes));
     encode_assign_kernel<false><<<blocks, EN_THREADS, EnSmem::bytes, st>>>(tm, int(n_centroids),
                                                                           static_cast<const __half*>(d_tokens), n_tokens,
-                                                                          d_codes, n_ctiles, nullptr);
+                                                                          d_codes, n_ctiles, nullptr, nullptr);
   }
   FPB_LAUNCH_CHECK("encode_assign");
   return FPB_OK;
@@ -360,8 +367,25 @@ extern "C" int fpb_kmeans_assign(int device, int dim, int64_t n_centroids, const
   }
   if (n_points == 0) return FPB_OK;
   FPB_CUDA_CHECK(cudaSetDevice(device));
-  return launch_assign(device, n_centroids, d_centroids, d_points, n_points, d_assign, d_bias,
+  return launch_assign(device, n_centroids, d_centroids, d_points, n_points, d_assign, d_bias, nullptr,
                        static_cast<cudaStream_t>(stream), "fpb_kmeans_assign");
+}
+
+extern "C" int fpb_nearest_centroid(int device, int dim, int64_t n_centroids, const void* d_centroids,
+                                    const float* d_bias, const void* d_points, int64_t n_points, int32_t* d_assign,
+                                    float* d_best, void* stream) {
+  if (dim != 128) {
+    fpb_set_error("fpb_nearest_centroid: this build handles dim=128 (got %d)", dim);
+    return FPB_ERR_UNSUPPORTED;
+  }
+  if (!d_centroids || !d_bias || !d_points || !d_assign || !d_best || n_centroids < 1 || n_points < 0) {
+    fpb_set_error("fpb_nearest_centroid: bad arguments");
+    return FPB_ERR_INVALID;
+  }
+  if (n_points == 0) return FPB_OK;
+  FPB_CUDA_CHECK(cudaSetDevice(device));
+  return launch_assign(device, n_centroids, d_centroids, d_points, n_points, d_assign, d_bias, d_best,
+                       static_cast<cudaStream_t>(stream), "fpb_nearest_centroid");
 }
 
 extern "C" int fpb_kmeans_update(int device, int dim, int64_t n_centroids, const void* d_points,
@@ -398,7 +422,8 @@ extern "C" int fpb_encode(int device, int nbits, int dim, int64_t n_centroids, c
   FPB_CUDA_CHECK(cudaSetDevice(device));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   {
-    const int rc = launch_assign(device, n_centroids, d_centroids, d_tokens, n_tokens, d_codes, nullptr, st, "fpb_encode");
+    const int rc = launch_assign(device, n_centroids, d_centroids, d_tokens, n_tokens, d_codes, nullptr, nullptr, st,
+                                 "fpb_encode");
     if (rc != FPB_OK) return rc;
   }
   const int pd = dim * nbits / 8;

@@ -133,6 +133,7 @@ EXPORTED_SYMBOLS = [
     "fpb_encode",
     "fpb_kmeans_assign",
     "fpb_kmeans_update",
+    "fpb_nearest_centroid",
     "fpb_cast_f32_to_f16_host",
     "fpb_cast_f32_to_f16_host_portable",
 ]
@@ -231,6 +232,8 @@ def load_library() -> ctypes.CDLL:
         lib.fpb_kmeans_assign.argtypes = [i32, i32, i64, vp, vp, vp, i64, vp, vp]
         lib.fpb_kmeans_update.restype = i32
         lib.fpb_kmeans_update.argtypes = [i32, i32, i64, vp, vp, vp, vp, vp, vp]
+        lib.fpb_nearest_centroid.restype = i32
+        lib.fpb_nearest_centroid.argtypes = [i32, i32, i64, vp, vp, vp, i64, vp, vp, vp]
         lib.fpb_token_scores.restype = i32
         lib.fpb_token_scores.argtypes = [vp, vp, i32, vp, vp, i32, i64, vp, vp]
         _lib = lib
@@ -327,6 +330,37 @@ def kmeans_assign(points: torch.Tensor, centroids: torch.Tensor) -> torch.Tensor
                                      bias.data_ptr(), points.data_ptr(), int(points.shape[0]), out.data_ptr(),
                                      torch.cuda.current_stream(dev).cuda_stream))
     return out
+
+
+def nearest_centroid(points: torch.Tensor, centroids: torch.Tensor,
+                     chunk: int = 4_000_000) -> tuple[torch.Tensor, torch.Tensor]:
+    """Nearest centroid and squared distance to it of every point [n, 128] (fpb_nearest_centroid; the outlier search
+    of update_centroids, update.py:121-150): (assign int32 [n], min_dist2 f32 [n]) on the centroids' CUDA device.
+
+    The points are taken as fp16; min_dist2 = |x|^2 - 2 max_k (<x, c_k> - |c_k|^2 / 2) with |x|^2 summed in fp32 from
+    the fp16 point and the dot products accumulated in fp32 on the tensor cores.  Host-resident points are streamed
+    to the device `chunk` rows at a time."""
+    _require_cuda()
+    lib = load_library()
+    dev = centroids.device
+    if dev.type != "cuda":
+        raise ValueError("nearest_centroid: the centroids must be on a CUDA device")
+    centroids = centroids.to(torch.float16).contiguous()
+    bias = (-0.5 * (centroids.float() ** 2).sum(1)).contiguous()
+    n, dim = int(points.shape[0]), int(points.shape[1])
+    assign = torch.empty((n,), dtype=torch.int32, device=dev)
+    dist2 = torch.empty((n,), dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        for s in range(0, n, chunk):
+            x = points[s : s + chunk].to(device=dev, dtype=torch.float16).contiguous()
+            m = int(x.shape[0])
+            best = dist2[s : s + m]
+            _check(lib.fpb_nearest_centroid(dev.index, dim, int(centroids.shape[0]), centroids.data_ptr(),
+                                            bias.data_ptr(), x.data_ptr(), m, assign[s : s + m].data_ptr(),
+                                            best.data_ptr(), stream))
+            best.mul_(-2.0).add_((x.float() ** 2).sum(1))
+    return assign, dist2
 
 
 def kmeans_update(points: torch.Tensor, assign: torch.Tensor, centroids: torch.Tensor) -> tuple[torch.Tensor, torch.Tensor]:

@@ -1,16 +1,24 @@
 """Index mutation: append documents / delete documents (host-side, off the hot path).
 
-Kept from the reference (python/fast_plaid/search/update.py:206-452, rust/index/update.rs:30-473,
-rust/index/delete.rs:26-145): create-if-missing, rebuild-from-scratch while the index is small
-and the raw ``embeddings.npy`` is still around, otherwise encode with the EXISTING codec and
-append; deletion rewrites the chunk files, renumbers the documents and rebuilds the IVF.
-Not reproduced (mutation policy, SURVEY.md section 2 rows 8/15): the outlier buffer and the
-centroid expansion of ``update_centroids``.
+The reference's update policy (python/fast_plaid/search/update.py:65-452, rust/index/update.rs:30-473,
+rust/index/delete.rs:26-145): create-if-missing; rebuild-from-scratch while the index is small and the
+raw ``embeddings.npy`` is still around; otherwise the outlier buffer.  Documents are appended with the
+existing codec and their raw embeddings kept in ``buffer.npy`` until ``buffer_size`` of them have
+accumulated; then the buffered documents are deleted, the tokens of buffer + new documents that lie
+farther than ``cluster_threshold`` from every centroid are clustered into new centroids appended to the
+codebook (``update_centroids``), all of them are re-added with the expanded codec and the threshold is
+re-estimated from their residuals.  Deletion rewrites the chunk files, renumbers the documents and
+rebuilds the IVF.
+
+The outlier search, min_k |x - c_k|^2 > threshold^2 over every token, runs on the tcgen05 nearest-centroid
+kernel (``engine.nearest_centroid``) on a CUDA device with dim 128, and as the reference's dense torch
+formula (update.py:144-150) elsewhere.
 """
 
 from __future__ import annotations
 
 import json
+import math
 import os
 from typing import Any
 
@@ -27,7 +35,7 @@ def _load_raw(path: str) -> list[torch.Tensor]:
 
 def process_update(fp: Any, docs: list[torch.Tensor], metadata: list[dict] | None, batch_size: int,
                    kmeans_niters: int, max_points_per_centroid: int, n_samples_kmeans: int | None, seed: int,
-                   start_from_scratch: int) -> None:
+                   start_from_scratch: int, buffer_size: int) -> None:
     index_path = fp.index
     meta = store.read_metadata(index_path)
     if meta is None:  # update.py:271-290
@@ -66,12 +74,110 @@ def process_update(fp: Any, docs: list[torch.Tensor], metadata: list[dict] | Non
         if len(old) + len(docs) > start_from_scratch and os.path.exists(emb_path):
             os.remove(emb_path)
         return
-    append_documents(index_path, docs, batch_size=batch_size, device=fp.devices[0])
+    from ..search.fast_plaid import save_list_tensors_on_disk
+
+    device = fp.devices[0]
+    buffer_path = os.path.join(index_path, "buffer.npy")
+    buffered = _load_raw(buffer_path) if os.path.exists(buffer_path) else []
+    if len(buffered) + len(docs) < buffer_size:  # update.py:431-445
+        save_list_tensors_on_disk(buffer_path, buffered + docs)
+        append_documents(index_path, docs, batch_size=batch_size, device=device)
+        return
+    # update.py:380-429: the buffered documents leave the index (their metadata rows stay: they come back with the
+    # same ids) and are re-added together with the new ones once the codebook has grown
+    if buffered:
+        fp._delete_documents(list(range(n_old - len(buffered), n_old)), delete_metadata=False, delete_buffer=False)
+        docs = buffered + docs
+    threshold = float(np.load(os.path.join(index_path, "cluster_threshold.npy")).item())
+    update_centroids(index_path, docs, threshold, device, kmeans_niters, max_points_per_centroid, seed,
+                     n_samples_kmeans)
+    if os.path.exists(buffer_path):
+        os.remove(buffer_path)
+    append_documents(index_path, docs, batch_size=batch_size, device=device, update_threshold=True)
 
 
 @torch.inference_mode()
-def append_documents(index_path: str, docs: list[torch.Tensor], batch_size: int, device: str) -> None:
-    """Encode with the codec on disk and append as new chunk(s) (update.rs:30-473)."""
+def outlier_mask(flat: torch.Tensor, centroids: torch.Tensor, cluster_threshold: float, device: str,
+                 rows: int = 4096) -> torch.Tensor:
+    """Host bool [n]: min_k |x - c_k|^2 > cluster_threshold^2 (update.py:121-150).
+
+    On CUDA with dim 128 the distances come from the tcgen05 kernel (fp16 tokens and centroids, fp32 accumulation).
+    Elsewhere they are the reference's x2 + y2 - 2 x.c in the tokens' dtype, in `rows`-row batches."""
+    dev = torch.device(device)
+    threshold_sq = cluster_threshold**2
+    if dev.type == "cuda" and flat.shape[1] == 128:
+        from ..engine import nearest_centroid
+
+        _, dist2 = nearest_centroid(flat, centroids.to(dev))
+        return (dist2 > threshold_sq).cpu()
+    cent = centroids.to(device=dev, dtype=flat.dtype)
+    y2 = torch.sum(cent**2, dim=1)
+    mask = torch.zeros(flat.shape[0], dtype=torch.bool)
+    for i in range(0, flat.shape[0], rows):
+        batch = flat[i : i + rows].to(dev)
+        x2 = torch.sum(batch**2, dim=1, keepdim=True)
+        dists_sq = x2 + y2 - 2 * torch.matmul(batch, cent.T)
+        mask[i : i + rows] = (torch.min(dists_sq, dim=1).values > threshold_sq).cpu()
+    return mask
+
+
+@torch.inference_mode()
+def update_centroids(index_path: str, docs: list[torch.Tensor], cluster_threshold: float, device: str,
+                     kmeans_niters: int, max_points_per_centroid: int, seed: int,
+                     n_samples_kmeans: int | None) -> None:
+    """Grow the codebook with k-means centroids of the outlier tokens (update.py:65-203).  Appends
+    ``k_update = max(1, 4 * ceil(n_outliers / max_points_per_centroid))`` centroids to ``centroids.npy`` (float32, as
+    the reference writes it), zero-length lists to ``ivf_lengths.npy`` and sets ``num_partitions``; without outliers
+    the directory is left untouched."""
+    centroids_path = os.path.join(index_path, "centroids.npy")
+    if not os.path.exists(centroids_path):
+        return
+    existing = np.load(centroids_path)
+    # the buffered documents come from disk, the new ones may be CUDA tensors
+    flat = torch.cat([d.reshape(-1, existing.shape[1]).to(device) for d in docs])
+    mask = outlier_mask(flat, torch.from_numpy(existing), cluster_threshold, device)
+    outliers = flat[mask.to(flat.device)]
+    n_out = int(outliers.shape[0])
+    if n_out == 0:
+        return
+    k_update = max(1, math.ceil(n_out / max_points_per_centroid) * 4)
+    new = build.compute_kmeans(outliers, int(outliers.shape[1]), device, kmeans_niters, max_points_per_centroid, seed,
+                               n_samples_kmeans, num_partitions=k_update)
+    new_np = new.detach().cpu().numpy().astype(np.float32)
+    final = np.concatenate([existing, new_np], axis=0)
+    np.save(centroids_path, final)
+    ivf_path = os.path.join(index_path, "ivf_lengths.npy")
+    if os.path.exists(ivf_path):
+        lengths = np.load(ivf_path)
+        np.save(ivf_path, np.concatenate([lengths, np.zeros(new_np.shape[0], dtype=lengths.dtype)]))
+    meta_path = os.path.join(index_path, "metadata.json")
+    with open(meta_path) as f:
+        meta = json.load(f)
+    meta["num_partitions"] = int(final.shape[0])
+    with open(meta_path, "w") as f:
+        json.dump(meta, f, indent=4)
+
+
+def updated_threshold(index_path: str, old_num_embeddings: int, residual_norms: torch.Tensor) -> None:
+    """update.rs:277-297: the 0.75 quantile of the appended tokens' residual norms, averaged with the stored threshold
+    weighted by token counts (the stored one counts the `old_num_embeddings` tokens the index held before the append);
+    written to ``cluster_threshold.npy`` as a float64 scalar."""
+    new_count = int(residual_norms.shape[0])
+    new_val = float(build._quantile_kth(residual_norms, 0.75))
+    path = os.path.join(index_path, "cluster_threshold.npy")
+    if os.path.exists(path):
+        old_val = float(np.load(path).item())
+        val = (old_val * old_num_embeddings + new_val * new_count) / (old_num_embeddings + new_count)
+    else:
+        val = new_val
+    np.save(path, np.array(val, dtype=np.float64))
+
+
+@torch.inference_mode()
+def append_documents(index_path: str, docs: list[torch.Tensor], batch_size: int, device: str,
+                     update_threshold: bool = False) -> None:
+    """Encode with the codec on disk and append as new chunk(s) (update.rs:30-473); with `update_threshold` the
+    cluster threshold is re-estimated from the appended tokens' residuals (update.rs:277-297)."""
     meta = store.read_metadata(index_path)
     nbits = int(meta["nbits"])
     dev = torch.device(device)
@@ -83,13 +189,17 @@ def append_documents(index_path: str, docs: list[torch.Tensor], batch_size: int,
     emb_offset = int(meta["num_embeddings"])
     n_docs = int(meta["num_documents"])
     per_chunk = max(1, int(batch_size))
+    norms: list[torch.Tensor] = []
     for s in range(0, len(docs), per_chunk):
         chunk_docs = docs[s : s + per_chunk]
         lens = [int(d.shape[0]) for d in chunk_docs]
-        flat = torch.cat([d.reshape(-1, dim).to(torch.float16) for d in chunk_docs]).to(dev)
+        flat = torch.cat([d.reshape(-1, dim).to(dev, torch.float16) for d in chunk_docs])
         codes_parts, res_parts = [], []
         for r in range(0, flat.shape[0], max(1, batch_size)):
-            c, rr = build.encode(flat[r : r + batch_size], cent, cent_t, cutoffs, nbits)
+            x = flat[r : r + batch_size]
+            c, rr = build.encode(x, cent, cent_t, cutoffs, nbits)
+            if update_threshold:  # fp32 norms of the fp16 residuals (update.rs:141-146)
+                norms.append((x - cent.index_select(0, c)).float().norm(dim=1).cpu())
             codes_parts.append(c.cpu())
             res_parts.append(rr.cpu())
         codes = torch.cat(codes_parts) if codes_parts else torch.empty(0, dtype=torch.int64)
@@ -98,6 +208,8 @@ def append_documents(index_path: str, docs: list[torch.Tensor], batch_size: int,
         n_chunks += 1
         emb_offset += int(codes.shape[0])
         n_docs += len(lens)
+    if norms:
+        updated_threshold(index_path, int(meta["num_embeddings"]), torch.cat(norms))
     compress_only = bool(meta.get("compress_only", False))
     if not compress_only:
         _rebuild_ivf(index_path, n_chunks, int(meta.get("num_partitions", cent.shape[0])), dev)

@@ -361,17 +361,19 @@ class FastPlaid:
         n_samples_kmeans: int | None = None,
         seed: int = 42,
         start_from_scratch: int = 999,
-        buffer_size: int = 100,  # noqa: ARG002
+        buffer_size: int = 100,
         use_triton_kmeans: bool | None = False,  # noqa: ARG002
     ) -> "FastPlaid":
-        """Add documents (fast_plaid.py:640-713, update.py:206-452).
+        """Add documents (fast_plaid.py:640-713, update.py:206-452), with the reference's policy.
 
-        Kept behaviour: create-if-missing; while the index holds at most ``start_from_scratch``
-        documents it is rebuilt from the raw ``embeddings.npy`` plus the new documents;
-        afterwards new documents are encoded with the existing codec and appended.  The
-        reference's centroid-expansion buffer (update.py:65-203) is an index-mutation policy
-        outside the search hot path and is not reproduced: appended documents always use the
-        existing centroids.
+        Create-if-missing; while the index holds at most ``start_from_scratch`` documents it is
+        rebuilt from the raw ``embeddings.npy`` plus the new documents.  Afterwards new documents
+        are encoded with the existing codec and appended, and their raw embeddings are kept in
+        ``buffer.npy``.  Once the buffer and the new documents reach ``buffer_size`` documents the
+        buffered ones are deleted, the tokens farther than the cluster threshold from every
+        centroid are clustered into new centroids appended to the codebook (update.py:65-203),
+        all of them are re-added with the expanded codec, the threshold is re-estimated from
+        their residuals and the buffer is removed.  ``use_triton_kmeans`` is accepted and ignored.
         """
         from ..index import update as _update
 
@@ -380,48 +382,52 @@ class FastPlaid:
             if isinstance(docs, torch.Tensor):
                 docs = list(docs) if docs.dim() == 3 else [docs]
             _update.process_update(self, docs, metadata, batch_size, kmeans_niters, max_points_per_centroid,
-                                   n_samples_kmeans, seed, start_from_scratch)
+                                   n_samples_kmeans, seed, start_from_scratch, buffer_size)
             self._swap_in_fresh()
         return self
 
     @torch.inference_mode()
     def delete(self, subset: list[int], _delete_metadata: bool = True, _delete_buffer: bool = True) -> "FastPlaid":  # noqa: ARG002
         """Remove documents and renumber the rest (fast_plaid.py:1045-1157, delete.rs:26-145)."""
-        from ..index import update as _update
-
         with self.lock:
-            # an index last updated by the reference may carry its buffer of recent raw documents (the most recent
-            # ones, fast_plaid.py:1084-1091): trim it like the reference does (:1118-1145) so that a later update by
-            # either implementation does not resurrect deleted documents
-            buffer_path = os.path.join(self.index, "buffer.npy")
-            if os.path.exists(buffer_path) and _delete_buffer:
-                n_docs = read_num_documents(self.index)
-                buf = np.load(buffer_path, allow_pickle=True)
-                start = n_docs - len(buf)
-                drop_b = {i - start for i in subset if start <= i < n_docs}
-                if drop_b:
-                    keep_b = [torch.from_numpy(buf[i]) for i in range(len(buf)) if i not in drop_b]
-                    if keep_b:
-                        save_list_tensors_on_disk(buffer_path, keep_b)
-                    else:
-                        os.remove(buffer_path)
-            _update.delete_from_index(self.index, subset, device=self.devices[0])
-            if os.path.exists(os.path.join(self.index, "metadata.db")) and _delete_metadata:
-                from ..filtering import delete as _meta_delete
-
-                _meta_delete(index=self.index, subset=subset)
-            emb_path = os.path.join(self.index, "embeddings.npy")
-            if os.path.exists(emb_path):
-                arr = np.load(emb_path, allow_pickle=True)
-                drop = {i for i in subset if i < len(arr)}
-                if drop:
-                    keep = [torch.from_numpy(arr[i]) for i in range(len(arr)) if i not in drop]
-                    if keep:
-                        save_list_tensors_on_disk(emb_path, keep)
-                    else:
-                        os.remove(emb_path)
+            self._delete_documents(subset, _delete_metadata, _delete_buffer)
             self._swap_in_fresh()
         return self
+
+    def _delete_documents(self, subset: list[int], delete_metadata: bool, delete_buffer: bool) -> None:
+        """The directory side of ``delete`` (the caller holds the lock and reloads the index afterwards)."""
+        from ..index import update as _update
+
+        # the buffer holds the raw embeddings of the most recent documents (fast_plaid.py:1084-1091): trim it like the
+        # reference does (:1118-1145) so that a later update by either implementation does not resurrect deleted
+        # documents
+        buffer_path = os.path.join(self.index, "buffer.npy")
+        if os.path.exists(buffer_path) and delete_buffer:
+            n_docs = read_num_documents(self.index)
+            buf = np.load(buffer_path, allow_pickle=True)
+            start = n_docs - len(buf)
+            drop_b = {i - start for i in subset if start <= i < n_docs}
+            if drop_b:
+                keep_b = [torch.from_numpy(buf[i]) for i in range(len(buf)) if i not in drop_b]
+                if keep_b:
+                    save_list_tensors_on_disk(buffer_path, keep_b)
+                else:
+                    os.remove(buffer_path)
+        _update.delete_from_index(self.index, subset, device=self.devices[0])
+        if os.path.exists(os.path.join(self.index, "metadata.db")) and delete_metadata:
+            from ..filtering import delete as _meta_delete
+
+            _meta_delete(index=self.index, subset=subset)
+        emb_path = os.path.join(self.index, "embeddings.npy")
+        if os.path.exists(emb_path):
+            arr = np.load(emb_path, allow_pickle=True)
+            drop = {i for i in subset if i < len(arr)}
+            if drop:
+                keep = [torch.from_numpy(arr[i]) for i in range(len(arr)) if i not in drop]
+                if keep:
+                    save_list_tensors_on_disk(emb_path, keep)
+                else:
+                    os.remove(emb_path)
 
     # ------------------------------------------------------------------ search
     def _loaded_indices(self) -> dict[str, Any]:

@@ -327,6 +327,14 @@ int fpb_kmeans_assign(int device, int dim, int64_t n_centroids, const void* d_ce
 int fpb_kmeans_update(int device, int dim, int64_t n_centroids, const void* d_points, const int64_t* d_order,
                       const int64_t* d_seg_offsets, void* d_centroids, float* d_shift, void* stream);
 
+/* ---- index update: outlier search of the centroid expansion (python/fast_plaid/search/update.py:121-150) ----
+ * fpb_nearest_centroid : the fpb_kmeans_assign argmax, plus d_best f32 [n] = the maximum itself,
+ *                        max_k (<x_i, c_k> + bias[k]) accumulated in fp32.  With bias[k] = -|c_k|^2 / 2 the caller
+ *                        gets min_k |x_i - c_k|^2 = |x_i|^2 - 2 d_best[i], which update_centroids compares with the
+ *                        squared cluster threshold.  dim 128 only (FPB_ERR_UNSUPPORTED otherwise). */
+int fpb_nearest_centroid(int device, int dim, int64_t n_centroids, const void* d_centroids, const float* d_bias,
+                         const void* d_points, int64_t n_points, int32_t* d_assign, float* d_best, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
