@@ -13,28 +13,23 @@ typedef CUresult (*fpb_encode_tiled_fn)(CUtensorMap*, CUtensorMapDataType, cuuin
                                         CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion,
                                         CUtensorMapFloatOOBfill);
 
-static int make_centroid_tmap(fpb_index* ix) {
-  ix->has_tmap = 0;
-  if (ix->dim != 128) return 0;
+const char* encode_centroid_tmap(CUtensorMap* tm, const void* d_centroids, int64_t K) {
   void* fn = nullptr;
   cudaDriverEntryPointQueryResult qres;
   if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess || !fn ||
       qres != cudaDriverEntryPointSuccess) {
     cudaGetLastError();
-    return 0;
+    return "cuTensorMapEncodeTiled is not available from this driver";
   }
-  static_assert(sizeof(CUtensorMap) == 128, "CUtensorMap is 128 bytes");
-  CUtensorMap* tm = reinterpret_cast<CUtensorMap*>(ix->tmap_centroids);
-  const cuuint64_t gdim[2] = {cuuint64_t(ix->dim), cuuint64_t(ix->K)};
-  const cuuint64_t gstride[1] = {cuuint64_t(ix->dim) * 2};
+  const cuuint64_t gdim[2] = {128, cuuint64_t(K)};
+  const cuuint64_t gstride[1] = {128 * 2};
   const cuuint32_t box[2] = {64, 128};
   const cuuint32_t estr[2] = {1, 1};
   const CUresult r = reinterpret_cast<fpb_encode_tiled_fn>(fn)(
-      tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<__half*>(ix->centroids), gdim, gstride, box, estr,
+      tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(d_centroids), gdim, gstride, box, estr,
       CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
       CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r == CUDA_SUCCESS) ix->has_tmap = 1;
-  return 0;
+  return r == CUDA_SUCCESS ? nullptr : "cuTensorMapEncodeTiled failed";
 }
 
 static thread_local char g_err[512] = "";
@@ -144,7 +139,10 @@ extern "C" int fpb_index_create(fpb_index** out, int device, int nbits, int dim,
       return rc != FPB_OK ? rc : FPB_ERR_CUDA;
     }
   }
-  make_centroid_tmap(ix);
+  // without a tensor map K1 runs the mma.sync kernel
+  static_assert(sizeof(CUtensorMap) == sizeof(ix->tmap_centroids), "CUtensorMap is 128 bytes");
+  ix->has_tmap =
+      dim == 128 && !encode_centroid_tmap(reinterpret_cast<CUtensorMap*>(ix->tmap_centroids), d_centroids, n_centroids);
   *out = ix;
   return FPB_OK;
 }

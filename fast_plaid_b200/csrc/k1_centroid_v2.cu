@@ -17,99 +17,38 @@
 // w / 4 of the 128-centroid tile), warp 8 issues the MMAs, warp 9 is the TMA producer.  (With four
 // epilogue warps the epilogue -- 128 conversions + stores per thread and tile -- was the critical
 // path: 0.33 ms.)
-#include <cuda.h>
 #include <string.h>
 
 #include "kernels.h"
+#include "tc05.cuh"
 
 namespace {
 
 constexpr int G1_THREADS = 320;
 constexpr int G1_PRODUCER_WARP = 9;
-constexpr int G1_STAGES = 3;
-constexpr int G1_KBLOCK = 128 * 128;      // bytes: 128 rows x 128 B
-constexpr int G1_TILE = 2 * G1_KBLOCK;    // 32 KB operand tile (K = 128)
 constexpr int G1_STAGING = 128 * 128 * 2;  // 32 KB fp16 output tile
-constexpr int G1_TMEM_COLS = 256;
 
 struct G1Smem {
   static constexpr int a_off = 0;
-  static constexpr int b_off = G1_TILE;
-  static constexpr int st_off = b_off + G1_STAGES * G1_TILE;
+  static constexpr int b_off = CT_TILE;
+  static constexpr int st_off = b_off + CT_STAGES * CT_TILE;
   static constexpr int bar_off = st_off + 2 * G1_STAGING;
   static constexpr int pmax_off = bar_off + 256;               // fp32 [128] partial tile maxima of the upper half
   static constexpr int bytes = pmax_off + 512 + 1024;
 };
 
-__device__ __forceinline__ void g1_mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void g1_mbar_arrive(uint32_t bar) {
-  asm volatile("{\n.reg .b64 st;\nmbarrier.arrive.shared::cta.b64 st, [%0];\n}" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void g1_mbar_wait(uint32_t bar, uint32_t parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred P1;\n"
-      "LAB_WAIT:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1;\n"
-      "@P1 bra DONE;\n"
-      "bra LAB_WAIT;\n"
-      "DONE:\n"
-      "}" ::"r"(bar),
-      "r"(parity)
-      : "memory");
-}
-__device__ __forceinline__ uint64_t g1_desc(uint32_t smem_addr) {
-  return uint64_t((smem_addr >> 4) & 0x3FFFu) | (uint64_t(1) << 16) | (uint64_t(1024 >> 4) << 32) |
-         (uint64_t(1) << 46) | (uint64_t(2) << 61);
-}
-__device__ __forceinline__ void g1_umma(uint32_t tmem_d, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
-                                        uint32_t accumulate) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "setp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n"
-      "}" ::"r"(tmem_d),
-      "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void g1_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void g1_tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-        "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]),
-        "=r"(r[16]), "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]),
-        "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
-// 16-byte chunk c (0..15) of row r of a [128 x 128] fp16 operand tile, K-major SWIZZLE_128B
-__device__ __forceinline__ uint32_t g1_sw_off(int r, int c) {
-  return uint32_t((c >> 3) * G1_KBLOCK + (r >> 3) * 1024 + (r & 7) * 128 + (((c & 7) ^ (r & 7)) << 4));
-}
-
 __global__ void __launch_bounds__(G1_THREADS, 1)
 k1_centroid_v2_kernel(const __grid_constant__ CUtensorMap tmap_c, int K, const __half* __restrict__ Qpad, int B, int Qp,
                       __half* __restrict__ S, __half* __restrict__ tmax, int n_ctiles, int tiles_per_split) {
   extern __shared__ unsigned char smem_dyn[];
-  const uint32_t dyn_addr = smem_u32(smem_dyn);
-  unsigned char* base = smem_dyn + ((1024u - (dyn_addr & 1023u)) & 1023u);
+  unsigned char* base = SMEM_ALIGN1024(smem_dyn);
   unsigned char* smA = base + G1Smem::a_off;
   unsigned char* smB = base + G1Smem::b_off;
   unsigned char* smS = base + G1Smem::st_off;
   uint64_t* bars = reinterpret_cast<uint64_t*>(base + G1Smem::bar_off);
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 16);
   float* pmax = reinterpret_cast<float*>(base + G1Smem::pmax_off);
-  const uint32_t bar_full = smem_u32(bars), bar_empty = smem_u32(bars + 3);
-  const uint32_t bar_tfull = smem_u32(bars + 6), bar_tempty = smem_u32(bars + 8);
+  const CtileBars ring(bars);
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int tt = blockIdx.x;                      // token tile
@@ -123,75 +62,24 @@ k1_centroid_v2_kernel(const __grid_constant__ CUtensorMap tmap_c, int K, const _
     const int tok = tt * 128 + r;
     uint4 v = make_uint4(0u, 0u, 0u, 0u);
     if (tok < n_tokens) v = *reinterpret_cast<const uint4*>(Qpad + int64_t(tok) * 128 + c * 8);
-    *reinterpret_cast<uint4*>(smA + g1_sw_off(r, c)) = v;
+    *reinterpret_cast<uint4*>(smA + sw128_off(r, c)) = v;
   }
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-  if (tid == 0) {
-    for (int s = 0; s < G1_STAGES; ++s) {
-      g1_mbar_init(bar_full + 8 * s, 1);
-      g1_mbar_init(bar_empty + 8 * s, 1);
-    }
-    for (int t = 0; t < 2; ++t) {
-      g1_mbar_init(bar_tfull + 8 * t, 1);
-      g1_mbar_init(bar_tempty + 8 * t, 8);
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 8) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "n"(G1_TMEM_COLS));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  fence_proxy_async();
+  if (tid == 0) ring.init(8);
+  if (warp == 8) tmem_alloc<CT_TMEM_COLS>(smem_u32(tmem_slot));
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   const int n_my = ct_end - ct_begin;
 
   if (warp == G1_PRODUCER_WARP) {
     // =========================== TMA producer: centroid tiles -> swizzled smem ===========================
-    if (lane == 0) {
-      for (int i = 0; i < n_my; ++i) {
-        const int stage = i % G1_STAGES;
-        g1_mbar_wait(bar_empty + 8 * stage, ((i / G1_STAGES) & 1) ^ 1);
-        const int k0 = (ct_begin + i) * 128;
-        const uint32_t dst = smem_u32(smB + stage * G1_TILE);
-        const uint32_t bar = bar_full + 8 * stage;
-        asm volatile("{\n.reg .b64 st;\nmbarrier.arrive.expect_tx.shared::cta.b64 st, [%0], %1;\n}" ::"r"(bar),
-                     "r"(uint32_t(G1_TILE))
-                     : "memory");
-#pragma unroll
-        for (int kb = 0; kb < 2; ++kb) {
-          asm volatile(
-              "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::
-                  "r"(dst + kb * G1_KBLOCK),
-              "l"(&tmap_c), "r"(kb * 64), "r"(k0), "r"(bar)
-              : "memory");
-        }
-      }
-    }
+    if (lane == 0) ctile_produce(&tmap_c, ring, smB, ct_begin, n_my, 0);
     __syncwarp();
   } else if (warp == 8) {
     // =========================== MMA issuer ===========================
-    if (lane == 0) {
-      const uint32_t a_addr = smem_u32(smA);
-      const uint32_t idesc = (1u << 4) | (uint32_t(128 >> 3) << 17) | (uint32_t(128 >> 4) << 24);
-      for (int i = 0; i < n_my; ++i) {
-        const int stage = i % G1_STAGES, acc = i & 1;
-        g1_mbar_wait(bar_full + 8 * stage, (i / G1_STAGES) & 1);
-        g1_mbar_wait(bar_tempty + 8 * acc, ((i >> 1) & 1) ^ 1);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        const uint32_t b_addr = smem_u32(smB + stage * G1_TILE);
-        const uint32_t d_tmem = tmem_base + acc * 128;
-#pragma unroll
-        for (int ks = 0; ks < 8; ++ks) {
-          const uint32_t off = (ks >> 2) * G1_KBLOCK + (ks & 3) * 32;
-          g1_umma(d_tmem, g1_desc(a_addr + off), g1_desc(b_addr + off), idesc, ks > 0 ? 1u : 0u);
-        }
-        g1_commit(bar_empty + 8 * stage);
-        g1_commit(bar_tfull + 8 * acc);
-      }
-    }
+    if (lane == 0) ctile_mma(ring, smA, smB, tmem_base, n_my, 0);
     __syncwarp();
   } else if (warp < 8) {
     // =========================== epilogue ===========================
@@ -212,26 +100,25 @@ k1_centroid_v2_kernel(const __grid_constant__ CUtensorMap tmap_c, int K, const _
       // the bulk stores issued from this staging buffer two tiles ago must have finished reading it
       if (tid < n_blk) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
       asm volatile("bar.sync 1, 256;" ::: "memory");
-      g1_mbar_wait(bar_tfull + 8 * acc, (i >> 1) & 1);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      mbar_wait(ring.tfull + 8 * acc, (i >> 1) & 1);
+      tc_fence_after();
       float mx = -INFINITY;
       unsigned char* my = stg + blk * blk_bytes + q * 2;
 #pragma unroll 1
       for (int c0 = 64 * half; c0 < 64 * half + 64; c0 += 32) {
-        uint32_t r[32];
-        g1_tmem_ld32(tmem_base + (uint32_t(quarter * 32) << 16) + acc * 128 + c0, r);
+        float v[32];
+        tmem_ld32(tmem_base + (uint32_t(quarter * 32) << 16) + acc * 128 + c0, v);
 #pragma unroll
         for (int x = 0; x < 32; ++x) {
-          const float f = __uint_as_float(r[x]);
-          if (c0 + x < rows_valid) mx = fmaxf(mx, f);
-          *reinterpret_cast<__half*>(my + (c0 + x) * (Qp * 2)) = __float2half_rn(f);
+          if (c0 + x < rows_valid) mx = fmaxf(mx, v[x]);
+          *reinterpret_cast<__half*>(my + (c0 + x) * (Qp * 2)) = __float2half_rn(v[x]);
         }
       }
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+      tc_fence_before();
       __syncwarp();
-      if (lane == 0) g1_mbar_arrive(bar_tempty + 8 * acc);
+      if (lane == 0) mbar_arrive(ring.tempty + 8 * acc);
       if (half == 1) pmax[trow] = mx;
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+      fence_proxy_async();
       asm volatile("bar.sync 1, 256;" ::: "memory");
       if (half == 0 && tok_valid)
         tmax[(int64_t(b) * Qp + q) * n_ctiles + ct] = __float2half_rn(fmaxf(mx, pmax[trow]));
@@ -250,11 +137,11 @@ k1_centroid_v2_kernel(const __grid_constant__ CUtensorMap tmap_c, int K, const _
     if (tid < n_blk) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
   }
 
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
   if (warp == 8) {
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(G1_TMEM_COLS));
+    tc_fence_after();
+    tmem_dealloc<CT_TMEM_COLS>(tmem_base);
   }
 }
 

@@ -1,5 +1,7 @@
 // Internal launchers (one per pipeline stage).  All are asynchronous on `stream`.
 #pragma once
+#include <cuda.h>
+
 #include "common.cuh"
 
 struct Ws {
@@ -31,6 +33,10 @@ struct Ws {
   int32_t* work2() const { return reinterpret_cast<int32_t*>(base + L->off_work2); }
   unsigned long long* stats() const { return reinterpret_cast<unsigned long long*>(base + L->off_stats); }
 };
+
+// TMA descriptor of an fp16 [K, 128] centroid table: 2-D, box 64 x 128 (one SWIZZLE_128B K block of a 128-centroid
+// tile), SWIZZLE_128B, rows past K zero-filled.  Returns nullptr on success, else why no map could be made.
+const char* encode_centroid_tmap(CUtensorMap* tm, const void* d_centroids, int64_t K);
 
 int launch_pad_queries(const fpb_index* ix, const Ws& ws, const __half* d_queries, cudaStream_t st);
 int launch_centroid_scores(const fpb_index* ix, const Ws& ws, cudaStream_t st);   // K1 (dispatch)

@@ -1,6 +1,8 @@
-// tcgen05 / mbarrier PTX wrappers shared by the MaxSim kernels that run on the 5th-generation
-// tensor cores (k5_maxsim_v5.cu).
+// The one home of the tcgen05 / mbarrier / TMA PTX used by the kernels on the 5th-generation tensor cores
+// (k1_centroid_v2.cu, encode.cu, k5_maxsim_v5.cu), and the centroid-tile ring that K1 v2 and encode_assign share.
 #pragma once
+
+#include <cuda.h>
 
 #include "common.cuh"
 
@@ -8,8 +10,15 @@
 __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
 }
+// makes the mbarrier.init of this thread visible to the async proxy (TMA, tcgen05.commit)
+__device__ __forceinline__ void mbar_fence_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
   asm volatile("{\n.reg .b64 st;\nmbarrier.arrive.shared::cta.b64 st, [%0];\n}" ::"r"(bar) : "memory");
+}
+// arrive and add `bytes` to the transaction count the phase waits for
+__device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t bytes) {
+  asm volatile("{\n.reg .b64 st;\nmbarrier.arrive.expect_tx.shared::cta.b64 st, [%0], %1;\n}" ::"r"(bar), "r"(bytes)
+               : "memory");
 }
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
   asm volatile(
@@ -27,6 +36,27 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+
+// 2-D TMA tile load of the box at (x, y) into shared memory; completion is counted on `bar` in bytes
+__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* tmap, int x, int y, uint32_t bar) {
+  asm volatile(
+      "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::
+          "r"(dst),
+      "l"(tmap), "r"(x), "r"(y), "r"(bar)
+      : "memory");
+}
+
+// TMEM allocation of COLS columns (a power of 2 >= 32), issued by one whole warp; the base address is written to
+// shared memory at `slot`.  The permit is relinquished at once: one CTA per SM, nothing else allocates.
+template <int COLS>
+__device__ __forceinline__ void tmem_alloc(uint32_t slot) {
+  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(slot), "n"(COLS));
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+}
+template <int COLS>
+__device__ __forceinline__ void tmem_dealloc(uint32_t base) {
+  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(base), "n"(COLS));
+}
 
 // K-major, SWIZZLE_128B shared-memory matrix descriptor (cute::UMMA::SmemDescriptor): start address
 // and offsets in 16-byte units, LBO = 1 (unused for swizzled K-major), SBO = 1024 B between 8-row
@@ -78,4 +108,85 @@ __device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&v)[8]) {
   asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 #pragma unroll
   for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
+}
+
+// ---- shared-memory layout ----------------------------------------------------------------
+// The dynamic shared array `p` rounded up to 1024 B, the alignment of a SWIZZLE_128B atom (the kernels reserve
+// 1024 B of slack for it).  A macro because the same code in an inline function reorders the kernels' later
+// swizzled-address arithmetic and changes their register allocation.
+#define SMEM_ALIGN1024(p) ((p) + ((1024u - (smem_u32(p) & 1023u)) & 1023u))
+// Byte offset of 16-byte chunk c (0..15) of row r in a [128 x 128] fp16 operand tile, K-major SWIZZLE_128B:
+// two K blocks of 128 rows x 128 B, chunk (c % 8) xor (r % 8) inside the row.
+__device__ __forceinline__ uint32_t sw128_off(int r, int c) {
+  return uint32_t((c >> 3) * (128 * 128) + (r >> 3) * 1024 + (r & 7) * 128 + (((c & 7) ^ (r & 7)) << 4));
+}
+
+// ---- centroid-tile ring (K1 v2, encode_assign) -------------------------------------------
+// A resident 128-token A tile against 128 x 128 fp16 centroid tiles that a TMA-producer lane streams through a
+// 3-stage shared-memory ring; an MMA-issuer lane accumulates each tile into one of two 128-column TMEM
+// accumulators, which an epilogue drains.  Ring iteration g (tiles this CTA streamed before) uses stage g % 3 and
+// accumulator g % 2.
+constexpr int CT_STAGES = 3;
+constexpr int CT_KBLOCK = 128 * 128;   // bytes: 128 rows x 128 B, one SWIZZLE_128B K block
+constexpr int CT_TILE = 2 * CT_KBLOCK;  // 32 KB operand tile (K = 128)
+constexpr int CT_TMEM_COLS = 256;       // two fp32 accumulators of 128 columns
+
+// Shared addresses of the ring's mbarriers, 10 consecutive uint64 from `bars`: full[3] (TMA -> MMA), empty[3]
+// (MMA -> TMA), tfull[2] (MMA -> epilogue), tempty[2] (epilogue -> MMA).
+struct CtileBars {
+  uint32_t full, empty, tfull, tempty;
+  __device__ __forceinline__ explicit CtileBars(const uint64_t* bars)
+      : full(smem_u32(bars)), empty(smem_u32(bars + 3)), tfull(smem_u32(bars + 6)), tempty(smem_u32(bars + 8)) {}
+  // one thread; tempty counts one arrival per epilogue warp
+  __device__ __forceinline__ void init(uint32_t epilogue_warps) const {
+    for (int s = 0; s < CT_STAGES; ++s) {
+      mbar_init(full + 8 * s, 1);
+      mbar_init(empty + 8 * s, 1);
+    }
+    for (int t = 0; t < 2; ++t) {
+      mbar_init(tfull + 8 * t, 1);
+      mbar_init(tempty + 8 * t, epilogue_warps);
+    }
+    mbar_fence_init();
+  }
+};
+
+// TMA producer (one lane): centroid tiles tile0 .. tile0 + n - 1 into ring iterations it .. it + n - 1.  Each
+// tile is two 64-column boxes; rows past K are zero-filled by the TMA unit.
+__device__ __forceinline__ void ctile_produce(const CUtensorMap* tmap, const CtileBars& bars, const unsigned char* smB,
+                                              int tile0, int n, uint32_t it) {
+  for (int i = 0; i < n; ++i) {
+    const uint32_t g = it + i;
+    const int stage = g % CT_STAGES;
+    mbar_wait(bars.empty + 8 * stage, ((g / CT_STAGES) & 1) ^ 1);
+    const uint32_t dst = smem_u32(smB + stage * CT_TILE);
+    const uint32_t bar = bars.full + 8 * stage;
+    mbar_arrive_expect_tx(bar, uint32_t(CT_TILE));
+#pragma unroll
+    for (int kb = 0; kb < 2; ++kb) tma_load_2d(dst + kb * CT_KBLOCK, tmap, kb * 64, (tile0 + i) * 128, bar);
+  }
+}
+
+// MMA issuer (one lane): ring iterations it .. it + n - 1, D[token][centroid] = A . B^T (M = N = K = 128) into
+// accumulator g % 2 at TMEM columns tmem_base + 128 (g % 2).
+__device__ __forceinline__ void ctile_mma(const CtileBars& bars, const unsigned char* smA, const unsigned char* smB,
+                                          uint32_t tmem_base, int n, uint32_t it) {
+  const uint32_t a_addr = smem_u32(smA);
+  const uint32_t idesc = umma_idesc(128);
+  for (int i = 0; i < n; ++i) {
+    const uint32_t g = it + i;
+    const int stage = g % CT_STAGES, acc = g & 1;
+    mbar_wait(bars.full + 8 * stage, (g / CT_STAGES) & 1);
+    mbar_wait(bars.tempty + 8 * acc, ((g >> 1) & 1) ^ 1);
+    tc_fence_after();
+    const uint32_t b_addr = smem_u32(smB + stage * CT_TILE);
+    const uint32_t d_tmem = tmem_base + acc * 128;
+#pragma unroll
+    for (int ks = 0; ks < 8; ++ks) {
+      const uint32_t off = (ks >> 2) * CT_KBLOCK + (ks & 3) * 32;
+      umma_f16(d_tmem, umma_desc(a_addr + off), umma_desc(b_addr + off), idesc, ks > 0 ? 1u : 0u);
+    }
+    umma_commit(bars.empty + 8 * stage);  // stage reusable once these MMAs have read it
+    umma_commit(bars.tfull + 8 * acc);    // accumulator ready
+  }
 }
