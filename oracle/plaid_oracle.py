@@ -189,6 +189,23 @@ def decompress_residuals(
     embedding_dimension: int,
     nbits: int,
 ) -> torch.Tensor:
+    emb = decode_unnormalised(packed_residuals, bucket_weights, byte_reversed_bits_map, bucket_weight_indices_lookup,
+                              codes, centroids, embedding_dimension, nbits)
+    norms = torch.linalg.vector_norm(emb, ord=2.0, dim=-1, keepdim=True).clamp_min(1e-12)  # :101-103
+    return emb / norms  # :105
+
+
+def decode_unnormalised(
+    packed_residuals: torch.Tensor,
+    bucket_weights: torch.Tensor,
+    byte_reversed_bits_map: torch.Tensor,
+    bucket_weight_indices_lookup: torch.Tensor,
+    codes: torch.Tensor,
+    centroids: torch.Tensor,
+    embedding_dimension: int,
+    nbits: int,
+) -> torch.Tensor:
+    """The decoded tokens before normalisation, e = fp16(w + c) (search.rs:66-99)."""
     n = codes.shape[0]
     packed_dim = (embedding_dimension * nbits) // 8  # :66
     per_byte = 8 // nbits  # :67
@@ -203,9 +220,7 @@ def decompress_residuals(
     gathered = bucket_weights.index_select(0, flat_bucket_idx.to(torch.int32))  # :91-92
     reshaped_w = gathered.view(n, packed_dim, per_byte)  # :93-94
     summed = reshaped_w + reshaped_centroids  # :97
-    emb = summed.view(n, embedding_dimension)  # :98-99
-    norms = torch.linalg.vector_norm(emb, ord=2.0, dim=-1, keepdim=True).clamp_min(1e-12)  # :101-103
-    return emb / norms  # :105
+    return summed.view(n, embedding_dimension)  # :98-99
 
 
 # --------------------------------------------------------------------------------------

@@ -116,6 +116,92 @@ def ranking_consistent(gpu_ids, gpu_scores, ref_score_of: dict, tol: float, fall
     return True, ""
 
 
+# ---- fp64 references with stated error bounds (DESIGN.md "Parity contract") -----------------------------------
+# Every rounding step of the search arithmetic is one IEEE operation, so each fp16 result the kernels produce must lie
+# in an interval around the exact (fp64) value: the fp32 error bound of the accumulation, widened outward to fp16.
+U32 = 2.0 ** -24  # unit roundoff of fp32
+# a dot product of at most 128 fp16 x fp16 products (each exact in fp32) accumulated in fp32: |err| <= 128 u sum|c q|
+DOT_TERMS = 128
+PAD_SENTINEL = -10000.0  # fp16(-9999), the score of a query token against a document without tokens
+
+
+def f16_step(h: torch.Tensor, direction: int) -> torch.Tensor:
+    """The fp16 neighbour of every entry of `h` (fp16) towards +inf (direction 1) or -inf (-1)."""
+    i = h.contiguous().view(torch.int16).to(torch.int32)
+    key = torch.where(i < 0, -(i & 0x7FFF), i) + direction  # order-preserving integer line, -0 and +0 both 0
+    bits = torch.where(key < 0, (-key) | 0x8000, key)
+    return torch.where(bits >= 0x8000, bits - 0x10000, bits).to(torch.int16).view(torch.float16)
+
+
+def round_down_f16(x: torch.Tensor) -> torch.Tensor:
+    """Largest fp16 <= x (x fp64)."""
+    h = x.half()
+    return torch.where(h.double() > x, f16_step(h, -1), h)
+
+
+def round_up_f16(x: torch.Tensor) -> torch.Tensor:
+    """Smallest fp16 >= x (x fp64)."""
+    h = x.half()
+    return torch.where(h.double() < x, f16_step(h, 1), h)
+
+
+def dot_fp64(a16: torch.Tensor, b16: torch.Tensor) -> tuple[torch.Tensor, torch.Tensor]:
+    """x = a . b^T in fp64 and gamma = 128 u sum|a b|, its fp32-accumulation bound ([n, D] x [m, D] -> [n, m])."""
+    a, b = a16.double(), b16.double()
+    return a @ b.T, DOT_TERMS * U32 * (a.abs() @ b.abs().T)
+
+
+def centroid_score_bounds(centroids16: torch.Tensor, q16: torch.Tensor) -> tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """fp16 [K, Q] interval [RD16(x - gamma), RU16(x + gamma)] every S[k, q] must lie in; also returns x and gamma."""
+    x, g = dot_fp64(centroids16, q16)
+    return round_down_f16(x - g), round_up_f16(x + g), x, g
+
+
+def interval_report(got: torch.Tensor, lo: torch.Tensor, hi: torch.Tensor, x: torch.Tensor, g: torch.Tensor) -> str:
+    """'' when lo <= got <= hi everywhere, else the count and the worst |got - x| / gamma among the violations."""
+    gd = got.double()
+    bad = (gd < lo.double()) | (gd > hi.double()) | torch.isnan(gd)
+    if not bool(bad.any()):
+        return ""
+    ratio = ((gd - x).abs() / g.clamp_min(1e-300))[bad]
+    return f"{int(bad.sum())} of {bad.numel()} entries outside the fp64 interval, worst |err| / gamma = {float(ratio.max()):.3g}"
+
+
+def token_norm_bounds(e16: torch.Tensor) -> tuple[torch.Tensor, torch.Tensor]:
+    """fp16 interval of fp16(sqrt(sum_fp32 e^2)) per row of e (fp16 [n, D]): the fp32 sum of the D exact squares is
+    within 128 u of the fp64 one, the square root adds one rounding."""
+    ss = (e16.double() ** 2).sum(-1)
+    lo = torch.sqrt(ss * (1 - DOT_TERMS * U32)) * (1 - U32)
+    hi = torch.sqrt(ss * (1 + DOT_TERMS * U32)) * (1 + U32)
+    return round_down_f16(lo), round_up_f16(hi)
+
+
+def normalise_like_the_kernels(e16: torch.Tensor, norms16: torch.Tensor) -> torch.Tensor:
+    """e_hat = fp16(fp32(e) / fp32(n)): one IEEE division (exact on the CPU), one rounding."""
+    return (e16.float() / norms16.float().unsqueeze(-1)).half()
+
+
+def maxsim_bounds(ehat16: torch.Tensor, offsets: list[int], lengths: list[int], q16: torch.Tensor,
+                  x: torch.Tensor | None = None, g: torch.Tensor | None = None) -> list[tuple[float, float]]:
+    """Interval [lo, hi] of the exact MaxSim score of each document (rows offsets[i] .. + lengths[i] of ehat16)
+    against the query q16 [Q, D]:  lo_q = RD16(max_t(x_tq - gamma_tq)),  hi_q = RU16(max_t(x_tq + gamma_tq)),
+    score in [sum lo_q - eps, sum hi_q + eps] with eps = Q u sum max(|lo_q|, |hi_q|) for the fp32 sum over q.
+    A document without tokens scores exactly Q * -10000 (lo == hi).  `x` / `g` may hold dot_fp64(ehat16, q16)."""
+    Q = q16.shape[0]
+    if x is None:
+        x, g = dot_fp64(ehat16, q16)
+    out = []
+    for o, n in zip(offsets, lengths):
+        if n == 0:
+            out.append((Q * PAD_SENTINEL, Q * PAD_SENTINEL))
+            continue
+        lo_q = round_down_f16((x[o : o + n] - g[o : o + n]).max(0).values).double()
+        hi_q = round_up_f16((x[o : o + n] + g[o : o + n]).max(0).values).double()
+        eps = Q * U32 * float(torch.maximum(lo_q.abs(), hi_q.abs()).sum())
+        out.append((float(lo_q.sum()) - eps, float(hi_q.sum()) + eps))
+    return out
+
+
 def merge_records_host(records: list[tuple[float, float, int]], R: int, top_k: int) -> list[tuple[int, float]]:
     """Host statement of the sharded merge rule (k6_merge_kernel): keep the R best by
     (approx desc, doc id asc), order them by (exact desc, doc id asc), emit top_k."""
